@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # jiminy_b200 on N B200s of one node
     python bench.py --impl reference --steps K --warmup W    # the CPU restatement of the reference path
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed
+
+The inputs are seeded: two runs with the same arguments step the same envs with the same actions, so the dumps
+of two builds of the project can be compared array for array.
 
 A "step" is one `Engine::step(0.04)` of every env of the batch -- for the default workload 4096
 PD-controlled ANYmal envs per GPU with spring-damper ground contact, RK4 at dtMax = 1 ms (160 full
@@ -159,6 +163,29 @@ def kernel_source_sha():
     return h.hexdigest()[:16]
 
 
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def step_outputs(eng):
+    """What a caller of `step` reads back after it (BatchedEngine or OracleBatch), one row per env, as float64 arrays."""
+    t, q, v, a = eng.get_state()
+    return {"t": t, "q": q, "v": v, "a": a, "sensors": eng.get_sensors(),
+            "status": eng.get_status().astype(np.float64), "env_index": np.arange(len(t), dtype=np.float64)}
+
+
+def dump_outputs(directory, outputs):
+    """Writes `outputs` as `<directory>/<name>.npy`.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of envs
+    (the same rows in every array, listed in `env_index`) is written instead, so that two builds compare row for row."""
+    n_env = len(outputs["env_index"])
+    row_bytes = sum(x[:1].nbytes for x in outputs.values())
+    if n_env * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n_env, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        outputs = {name: x[rows] for name, x in outputs.items()}
+    os.makedirs(directory, exist_ok=True)
+    for name, x in outputs.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.ascontiguousarray(x, dtype=np.float64))
+
+
 def run_reference(args):
     """`--impl reference`: times the reference's CPU implementation of the path.  The reference itself
     cannot be built in this image (Eigen / Boost / Pinocchio / hpp-fcl absent, no network), so this is
@@ -186,6 +213,8 @@ def run_reference(args):
         rc = orc.step(sc.step_dt, parallel=True)
         assert args.action == "torque" or not rc.any()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, step_outputs(orc))
     value = n_env * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -287,6 +316,8 @@ def run_gpu(args):
     barrier()
     eng.synchronize()       # PeerTimeout here = a signal of the timed region never arrived: no number is printed
     launches = eng.launch_count() - launches0
+    # read back before the arms below step the batch further: the dump is the state of the last timed step
+    outputs = step_outputs(eng) if args.dump_outputs and rank == 0 else None
     clocks = sampler.stop()
     kernel_ms = [a.elapsed_time(b) for (a, _), b in zip(ev, evk)]      # step kernel alone (roofline)
     step_ms = [a.elapsed_time(b) for a, b in ev]                        # step + observation all-gather
@@ -396,6 +427,8 @@ def run_gpu(args):
                                 "sample": f"{cpu['all_threads']['n_env']} envs x {cpu['all_threads']['steps']} env-steps, "
                                           f"OpenMP over envs ({cpu['all_threads']['seconds']:.1f} s)",
                                 "single_thread_value": cpu["single_thread"]["value"], "usable_cores": cpu["usable"], "note": PORT_NOTE}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -422,7 +455,12 @@ def main():
     ap.add_argument("--flagged-fraction", type=float, default=0.0,
                     help="PD mode: share of the envs driven through their hip joint bounds (stepped by the full body with joint-bound constraints)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the time, state, sensors and status of every env after the last timed step as "
+                         "DIR/<name>.npy (float64; a seeded sample of envs above 64 MB in all); multi-GPU: rank 0's envs")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -9,9 +9,10 @@ import pytest
 from jiminy_b200 import model as M
 from jiminy_b200 import robots as R
 
-from conftest import DATA
+from conftest import DATA, ROOT
 
-REF = "/root/reference/data"
+# the reference's ANYmal description (ANYbotics' anymal.urdf and jiminy's anymal_hardware.toml), kept as test inputs
+REF_ANYMAL = os.path.join(ROOT, "tests", "golden", "anymal")
 
 
 def test_simple_pendulum_fixed_joint_merge():
@@ -90,11 +91,10 @@ def test_atlas_contact_cleanup():
     assert r.contact_frame_names == sorted(r.contact_frame_names)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference data not available on this machine")
 def test_compiled_tables_match_reference_data():
     """The shipped JSON tables are what the compiler produces from the reference's data files."""
-    robot = M.build_robot_table(os.path.join(REF, "quadrupedal_robots/anymal/anymal.urdf"), True)
-    M.load_hardware_description_file(robot, os.path.join(REF, "quadrupedal_robots/anymal/anymal_hardware.toml"))
+    robot = M.build_robot_table(os.path.join(REF_ANYMAL, "anymal.urdf"), True)
+    M.load_hardware_description_file(robot, os.path.join(REF_ANYMAL, "anymal_hardware.toml"))
     shipped, _ = R.load_robot("anymal")
     np.testing.assert_array_equal(robot.placement, shipped.placement)
     np.testing.assert_array_equal(robot.inertia, shipped.inertia)
