@@ -572,8 +572,11 @@ int jb_batch_create(const JbModelDesc* m, const JbOptions* opt, int32_t n_env, i
 
 int jb_describe(JbBatch* b, char* buf, int32_t len) {
     if (!b || !buf) return fail(JB_ERR_INVALID_ARGUMENT, "null argument");
-    std::snprintf(buf, len, "%s; hot path: %s%s; constraints: %s", b->plan.describe().c_str(),
-                  b->kp.sig_id == SigQuadruped::ID ? (b->kp.rhs_variant == 1 ? "quadruped signature, composite-rigid-body evaluation" : "quadruped signature, ABA sweeps") : "ABA sweeps (dynamic plan)",
+    // (names every switch of the evaluation path, so that a test or an A/B run can check which one it measured)
+    const char* hot = b->no_fast_kernel ? "none, every step runs the full kernel"
+                      : b->kp.sig_id == SigQuadruped::ID ? (b->kp.rhs_variant == 1 ? "quadruped signature, composite-rigid-body evaluation" : "quadruped signature, ABA sweeps")
+                      : (b->kp.all_uniform ? "ABA sweeps (dynamic plan, lane-uniform descriptors)" : "ABA sweeps (dynamic plan, per-lane descriptors)");
+    std::snprintf(buf, len, "%s; hot path: %s%s; constraints: %s", b->plan.describe().c_str(), hot,
                   b->kp.fast_bounds ? ", joint bounds solved in the evaluation" : "",
                   !b->kp.cons_on ? "flag only" : (b->kp.cq_on ? (b->kp.lb_on ? "structured quadruped solver + lane-block solver" : "structured quadruped solver + generic")
                                                  : (b->kp.bd_on ? "body-space contact solver + lane-block solver" : (b->kp.lb_on ? "lane-block solver" : "generic solver"))));
